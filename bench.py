@@ -27,6 +27,8 @@ the reference: (root.visitSum - root.freeVisits) / elapsed (engine/src/evalinfo.
            simulations; cfg 3: chess RISEv3.3 Batch_Size 64, 1600 simulations) instead of the headline workload.
   --config 4|5: the self-play configurations (cfg 4: chess960, RISEv3.3, 8 concurrent games per GPU; cfg 5: King of the
            Hill + Three-check mixed, RISEv2 63 channels, Batch_Size 128 rows per forward): FINISHED games per hour.
+  --dump-outputs DIR: after the timed steps, the last step's search result (root moves, visits, Q, priors, MCTS policy,
+           principal variation, root scalars) as DIR/<name>.npy, for comparing two builds output for output.
 Multi-GPU: replicas only (games/searches never interact; no collective on the data path): every rank runs the same
 workload on its own GPU, value = sum of nodes / max over ranks of the time ("weak" scaling).
 """
@@ -364,6 +366,38 @@ def search_leg(agent, net, steps, flush):
     return nodes, dev_ms, wall_s, last
 
 
+# the EvalInfo fields of a search result that --dump-outputs writes, besides the root moves and the principal variation;
+# elapsed_ms and nps are timings, not results
+RESULT_ARRAYS = ("visits", "q", "prior", "policy")
+RESULT_SCALARS = ("root_value", "best_move_q", "visit_sum", "free_visits", "nodes", "best_idx", "node_type", "pv_len",
+                  "iterations", "evals", "tree_nodes", "nodes_pre_search", "sum_select_k", "sum_depth", "error")
+
+
+def dump_outputs(out_dir, result, variant_id):
+    """Writes a search result (the dict MCTSAgent.evaluate_board_state returns for the start position) as
+    out_dir/<name>.npy: the root's children in the search's order (moves as 16-bit move codes, visits, Q, priors, MCTS
+    policy), the principal variation as move codes, and every scalar of the result, so that two builds can be compared
+    output for output.  Q and priors stay float32, everything else is float64."""
+    import numpy as np
+
+    from crazyara_b200.engine import BoardState
+    os.makedirs(out_dir, exist_ok=True)
+    state = BoardState().set("", False, variant_id)
+    arrays = {"moves": np.array([state.uci_to_action(m) for m in result["moves"]], np.float64)}
+    pv = []
+    for m in result["pv"]:
+        pv.append(state.uci_to_action(m))
+        state.do_uci(m)
+    arrays["pv"] = np.array(pv, np.float64)
+    for name in RESULT_ARRAYS:
+        a = np.asarray(result[name])
+        arrays[name] = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+    for name in RESULT_SCALARS:
+        arrays[name] = np.array([result[name]], np.float32 if name in ("root_value", "best_move_q") else np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -380,7 +414,13 @@ def main():
     ap.add_argument("--trees", type=int, default=32, help="extra leg: concurrent searches per GPU (0 = skip)")
     ap.add_argument("--selfplay-seconds", type=float, default=8.0, help="extra leg: self-play arena window (0 = skip)")
     ap.add_argument("--selfplay-games", type=int, default=64)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the search result of the last one "
+                    "as DIR/<name>.npy (search configurations M, 2, 3 on the GPU)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config in ("4", "5")):
+        ap.error("--dump-outputs writes the GPU search result: --impl ours with --config M, 2 or 3")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -400,8 +440,7 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return
-        # the same workload, bounded so that the run ends within a few minutes (a 3200-simulation CPU search takes ~4 s)
-        steps = max(1, min(args.steps, 20))
+        steps = args.steps
         warm = min(args.warmup, 1)
         nps, ms, cores, kind, sample = cpu_arm(args.config, sims, batch, args.threads, steps, warm)
         print(json.dumps({
@@ -453,6 +492,8 @@ def main():
         dist.barrier()
     sampler.stop_flag = True
     sampler.join(timeout=2)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last, vid)
     launches = agent.launch_count() + net.launch_count() - launches0
     # phase split: CUDA events between the kernels of every iteration, which the timed searches above do without
     # (an iteration is a graph launch there) -- measured on extra searches

@@ -72,6 +72,29 @@ def golden_input(arch, n=4, seed=123):
     return x
 
 
+def _f32(a):
+    """float32 values as the shortest decimals that read back to the same float32."""
+    return [float(f"{x:.9g}") for x in np.asarray(a, np.float32).ravel()]
+
+
+def record_live_cases():
+    """tests/golden/net_reference_live.json: the reference module on state_dict seed 7 and three input positions (seed 9)
+    for the architectures test_oracle_net_matches_imported_reference checks; the logits at every 11th column plus the
+    sums over all columns."""
+    rec = {}
+    for name, arch in (("risev2_34", onet.arch_risev2(34, 81)), ("risev33_52", onet.arch_risev33(52, 76, True))):
+        sd = onet.make_state_dict(arch, 7)
+        value, logits, aux = reference_forward(arch, sd, golden_input(arch, n=3, seed=9))
+        idx = np.arange(0, logits.shape[1], 11)
+        rec[name] = dict(seed=7, input_seed=9, n=3, value=_f32(value), aux=None if aux is None else _f32(aux),
+                         logit_idx=idx.tolist(), logits=_f32(logits[:, idx]), logits_sum=logits.astype(np.float64).sum(1).tolist(),
+                         logits_abs_sum=np.abs(logits.astype(np.float64)).sum(1).tolist())
+    path = os.path.join(ROOT, "tests", "golden", "net_reference_live.json")
+    with open(path, "w") as f:
+        json.dump(rec, f, separators=(",", ":"))
+    print("wrote", path)
+
+
 def main():
     for arch in (onet.arch_risev2(34, 81), onet.arch_risev33(52, 76, True), onet.arch_risev2(63, 84)):
         sd = onet.make_state_dict(arch, seed=0)
@@ -88,6 +111,7 @@ def main():
         with open(path, "w") as f:
             json.dump(rec, f)
         print("wrote", path, "value", value)
+    record_live_cases()
 
 
 if __name__ == "__main__":

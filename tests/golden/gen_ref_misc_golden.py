@@ -4,6 +4,7 @@
 import ctypes
 import json
 import os
+import random
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
@@ -18,6 +19,18 @@ PGN_CASES = [
          moves=["e4", "e5", "Nf3", "Nc6", "Bb5", "a6", "Ba4", "Nf6", "O-O", "Be7", "Re1", "b5", "Bb3", "d6", "c3", "O-O",
                 "h3"]),
 ]
+
+
+def random_pgn_cases():
+    """Seeded games of 0 to 120 moves drawn from SAN spellings that exercise castling, promotions, drops and checks."""
+    rng = random.Random(5)
+    cases = []
+    for n in (0, 1, 2, 7, 8, 9, 16, 33, 120):
+        moves = [rng.choice(["e4", "Nf3", "O-O", "exd5", "Q@h5+", "a8Q", "Rad1", "N@f7#"]) for _ in range(n)]
+        header = ["crazyhouse960", "SelfPlay", "2026.09.24 10:00:00", "Darmstadt, GER", "?", "some fen", "x", "y",
+                  rng.choice(["1-0", "0-1", "1/2-1/2"]), "?"]
+        cases.append(dict(header=header, moves=moves))
+    return cases
 
 
 def render(L, case):
@@ -40,6 +53,8 @@ def main():
     tails = sorted({f.split("/", 1)[1].split("/", 6)[0] + "|" + f.split(" ", 1)[1] for f in fens})
     json.dump({"pgn": [dict(c, text=render(L, c)) for c in PGN_CASES], "chess960_back_ranks": ranks,
                "chess960_fen_shape": tails}, open(os.path.join(HERE, "ref_misc.json"), "w"), separators=(",", ":"))
+    json.dump({"text": [render(L, c) for c in random_pgn_cases()]}, open(os.path.join(HERE, "ref_pgn_random.json"), "w"),
+              separators=(",", ":"))
     print(len(ranks), "distinct chess960 set-ups,", len(PGN_CASES), "pgn cases")
 
 

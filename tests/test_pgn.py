@@ -97,20 +97,13 @@ def test_pgn_text_equals_the_reference_writer_golden():
 
 
 def test_pgn_text_equals_the_compiled_reference_live():
-    import ctypes
+    """Seeded random games (0 to 120 moves) against the text the compiled reference writer produced for them
+    (tests/golden/ref_pgn_random.json, recorded by tests/golden/gen_ref_misc_golden.py)."""
+    import json
     import os
-    import random
-    so = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "libref_parts.so")
-    if not os.path.exists(so):
-        pytest.skip("oracle/_ref not built on this box (no reference sources)")
-    L = ctypes.CDLL(so)
-    rng = random.Random(5)
-    for n in (0, 1, 2, 7, 8, 9, 16, 33, 120):
-        moves = [rng.choice(["e4", "Nf3", "O-O", "exd5", "Q@h5+", "a8Q", "Rad1", "N@f7#"]) for _ in range(n)]
-        header = ["crazyhouse960", "SelfPlay", "2026.09.24 10:00:00", "Darmstadt, GER", "?", "some fen", "x", "y",
-                  rng.choice(["1-0", "0-1", "1/2-1/2"]), "?"]
-        hdr = (ctypes.c_char_p * 10)(*[h.encode() for h in header])
-        mv = (ctypes.c_char_p * max(n, 1))(*[m.encode() for m in moves] or [b""])
-        out = ctypes.create_string_buffer(1 << 16)
-        assert L.ref_pgn_render(hdr, mv, n, out, 1 << 16) >= 0
-        assert str(_game_from(dict(header=header, moves=moves))) == out.value.decode()
+    from tests.golden.gen_ref_misc_golden import random_pgn_cases
+    g = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "ref_pgn_random.json")))
+    cases = random_pgn_cases()
+    assert len(cases) == len(g["text"]) == 9
+    for case, text in zip(cases, g["text"]):
+        assert str(_game_from(case)) == text

@@ -126,25 +126,13 @@ def test_time_for_move_equals_the_reference_golden():
 
 
 def test_time_for_move_equals_the_compiled_reference_live():
-    """The same against oracle/_ref/libref_parts.so itself on fresh random inputs, where the reference sources exist
-    (the build container); skipped on boxes without them."""
-    import ctypes
+    """The same on 5000 seeded random inputs, against what the compiled reference (oracle/_ref/libref_parts.so) returned
+    for them (tests/golden/timeman_random.json, recorded by tests/golden/gen_timeman_golden.py)."""
+    import json
     import os
-    import random
-    import subprocess
-    import pytest
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    so = os.path.join(root, "oracle", "_ref", "libref_parts.so")
-    if not os.path.exists(so):
-        if not os.path.isdir("/root/reference/engine/src"):
-            pytest.skip("no reference sources on this box")
-        subprocess.run(["make", "-s", "-C", os.path.join(root, "oracle"), "ref"], check=True)
-    R = ctypes.CDLL(so)
-    R.ref_time_for_move.argtypes = [ctypes.c_long] + [ctypes.c_int] * 8
-    rng = random.Random(11)
-    for _ in range(5000):
-        clock = rng.random() < 0.8
-        row = (0 if clock else rng.choice((0, 1, 30, 250, 4000)), rng.randrange(0, 3000000) if clock else 0,
-               rng.randrange(0, 3000000) if clock else 0, rng.randrange(0, 30000), rng.randrange(0, 30000),
-               rng.choice((0, 0, 0, 1, 7, 40)), rng.choice((0, 20, 100, 500)), rng.randrange(2), rng.randrange(1, 120))
-        assert _ara_time_for_move(row) == R.ref_time_for_move(*row), row
+    from tests.golden.gen_timeman_golden import random_rows
+    g = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "timeman_random.json")))
+    rows = random_rows()
+    assert len(rows) == len(g["reference_ms"]) == 5000
+    for row, ref_ms in zip(rows, g["reference_ms"]):
+        assert _ara_time_for_move(row) == ref_ms, row
